@@ -23,14 +23,14 @@ from sparkflow_b200.ops.layout import ParamLayout
 from sparkflow_b200.ops.optimizers import NUM_SLOTS, OPT_IDS, OptimizerSpec, apply_update, init_slots
 from sparkflow_b200.parallel.rwlock import RWLock
 
-FIXTURE = "/root/reference/tests/test_model/to_load"
-HAVE_FIXTURE = os.path.exists(FIXTURE + ".meta")
+# a TF-1.7 checkpoint (MetaGraphDef + V2 bundle, 2-10 tanh-10 tanh-1 sigmoid with Adam slots) written by the original
+# sparkflow test suite: the codec tests decode it and rewrite it byte for byte
+FIXTURE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "test_model", "to_load")
 
 
 # ---------------------------------------------------------------------------------------------
 # protobuf codec
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.skipif(not HAVE_FIXTURE, reason="reference fixture not mounted")
 def test_pbwire_decodes_real_tf_metagraph():
     mg = pbwire.decode("MetaGraphDef", open(FIXTURE + ".meta", "rb").read())
     assert len(mg["graphDef"]["node"]) == 264 and mg["metaInfoDef"]["tensorflowVersion"] == "1.7.0"
@@ -113,7 +113,7 @@ def test_interpreter_rejects_unknown_ops_loudly():
         prog.run(["weird:0"], {"x:0": np.zeros((1, 10), np.float32)}, {})
 
 
-def test_session_and_saver_roundtrip(tmp_path):
+def test_session_and_saver_roundtrip(tmp_path, monkeypatch):
     g = tf.Graph()
     with g.as_default():
         zoo.fixture_mlp()
@@ -130,7 +130,12 @@ def test_session_and_saver_roundtrip(tmp_path):
     from sparkflow_b200.ml_util import run_inference
 
     w = [np.asarray(a, np.float32) for a in json.loads(m.getOrDefault(m.modelWeights))]
-    np.testing.assert_allclose(run_inference(m.getOrDefault(m.modelJson), w, x, "x:0", "out/Sigmoid:0"), out1, rtol=1e-5, atol=1e-6)
+    args = (m.getOrDefault(m.modelJson), w, x, "x:0", "out/Sigmoid:0")
+    if torch.cuda.is_available():
+        # with a GPU, run_inference takes the compiled forward plan (bf16 operands); the session ran the fp32 interpreter
+        np.testing.assert_allclose(run_inference(*args), out1, rtol=1e-2, atol=1e-3)
+        monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
+    np.testing.assert_allclose(run_inference(*args), out1, rtol=1e-5, atol=1e-6)          # the fp32 interpreter path
 
 
 # ---------------------------------------------------------------------------------------------
@@ -293,7 +298,6 @@ def test_param_layout_tables():
     assert lay.tile_map().shape == (25 * 4 + 4 + 8 + 1, 3)
 
 
-@pytest.mark.skipif(not HAVE_FIXTURE, reason="reference fixture not mounted")
 def test_bundle_reader_and_writer_are_byte_exact(tmp_path):
     from sparkflow_b200.io.bundle import read_bundle, read_checkpoint_state, write_bundle
 
